@@ -53,6 +53,8 @@ def parse():
     ap.add_argument("--window-mib", type=int, default=16)
     ap.add_argument("--config", type=int, default=None, choices=[0, 1, 2, 3, 4],
                     help="shorthand for BASELINE.json configs[N] (0: 256 MiB no transform, 1: zstd, 2: aes, 3: zstd+aes, 4: ranged fetch)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_transform_outputs)")
     a = ap.parse_args()
     if a.config is not None:
         if a.config == 0:
@@ -61,6 +63,8 @@ def parse():
             a.workload, a.direction = "zstd+aes", "fetch"
         else:
             a.workload = {1: "zstd", 2: "aes", 3: "zstd+aes"}[a.config]
+    if a.dump_outputs and (a.impl != "tsgpu" or a.direction != "transform" or a.workload == "none"):
+        ap.error("--dump-outputs covers the GPU transform path only (--impl tsgpu, --direction transform, a transforming workload)")
     return a
 
 
@@ -517,6 +521,32 @@ def bind_to_gpu_numa_node(torch, index):
         pass
 
 
+DUMP_BUDGET = 60_000_000        # bytes of .npy payload: --dump-outputs stays under 64 MB whatever the segment size
+
+
+def dump_transform_outputs(path, d_slots, d_sizes, stride, nch):
+    """Writes what a caller of transform_device receives, so that two builds can be compared output for output:
+      transformed_sizes.npy  float64 [nch]     every chunk's transformed size (d_sizes)
+      sample_chunk_ids.npy   float64 [k]       a fixed, seeded sample of chunk indices (k from the budget and the slot size)
+      sample_chunks.npy      float32 [k, w]    those chunks' transformed bytes (the slot past SLOT_HEAD), zero past the chunk's end
+    The sample depends only on the shape arguments, never on what the path computed."""
+    from tsgpu import binding
+    os.makedirs(path, exist_ok=True)
+    sizes = d_sizes.cpu().numpy().astype(np.int64)
+    width = stride - binding.SLOT_HEAD
+    cols = min(width, (DUMP_BUDGET - 16 * nch) // 4)
+    k = max(1, min(nch, (DUMP_BUDGET - 16 * nch) // (4 * cols)))
+    ids = np.sort(np.random.default_rng(20240).choice(nch, k, replace=False))
+    chunks = np.zeros((k, cols), dtype=np.float32)
+    for j, i in enumerate(ids):
+        n = min(int(sizes[i]), cols)
+        a = int(i) * stride + binding.SLOT_HEAD
+        chunks[j, :n] = d_slots[a:a + n].cpu().numpy()
+    np.save(os.path.join(path, "transformed_sizes.npy"), sizes.astype(np.float64))
+    np.save(os.path.join(path, "sample_chunk_ids.npy"), ids.astype(np.float64))
+    np.save(os.path.join(path, "sample_chunks.npy"), chunks)
+
+
 def main_tsgpu(args):
     import torch
     import torch.distributed as dist
@@ -577,6 +607,8 @@ def main_tsgpu(args):
     ms = e0.elapsed_time(e1)
     launches = ctx.launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_transform_outputs(args.dump_outputs, d_slots, d_sizes, stride, nch)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -4,7 +4,8 @@
 Two kinds of content:
   reference_vectors.json   golden vectors TRANSCRIBED from the reference's own tests (values only; each entry cites
                            the file:line it was read from, T = core/src/test/java/io/aiven/kafka/tieredstorage) plus the
-                           public AES-256 GCM-specification / FIPS-197 known answers the AES path is pinned on.
+                           public AES-256 GCM-specification / FIPS-197 known answers the AES path is pinned on, and the
+                           declarations of the reference members the Java sources under jni/ use.
   libzstd_frames.json      frames GENERATED here by the oracle's libzstd (system libzstd, dlopen) from corpus.gen_chunk
                            inputs, at the level the reference uses (3) and at 1 / 19 for coverage, so that the decoder
                            parity tests do not depend on which libzstd the test box carries.  The reference is Java and
@@ -70,6 +71,20 @@ REFERENCE_VECTORS = {
         "source": "FIPS-197 Appendix C.3; public",
         "key": "000102030405060708090a0b0c0d0e0f101112131415161718191a1b1c1d1e1f",
         "pt": "00112233445566778899aabbccddeeff", "ct": "8ea2b7ca516745bfeafc49904b496089",
+    },
+    "java_api": {
+        "source": "declarations of the reference types / members jni/ names, transcribed from the reference's main sources "
+                  "(M = core/src/main/java/io/aiven/kafka/tieredstorage, S = storage/core/src/main/java/io/aiven/kafka/tieredstorage)",
+        "files": {
+            "M/Chunk.java": {"lines": "22-26", "declarations": [
+                "public final int id;", "public final int originalPosition;", "public final int originalSize;",
+                "public final int transformedPosition;", "public final int transformedSize;"]},
+            "M/manifest/SegmentEncryptionMetadata.java": {"lines": "24", "declarations": ["SecretKey dataKey();"]},
+            "M/fetch/ChunkManager.java": {"lines": "28", "declarations": ["InputStream getChunk(final ObjectKey objectKey,"]},
+            "M/transform/DetransformChunkEnumeration.java": {"lines": "28", "declarations": [
+                "public interface DetransformChunkEnumeration extends Enumeration<byte[]> {"]},
+            "S/storage/BytesRange.java": {"lines": "100", "declarations": ["public static BytesRange of(final int from, final int to) {"]},
+        },
     },
 }
 

@@ -116,8 +116,6 @@ def test_emulated_dense_frames_are_the_committed_ones():
 
 
 @pytest.mark.gpu
-@pytest.mark.xfail(strict=False, reason="emulator-vs-hardware byte identity of dense-mode frames: added after the round's last GPU "
-                                        "lease, so its first run on a B200 is the driver's; an XPASS is the expected outcome")
 def test_gpu_dense_frames_equal_the_emulators():
     # the B200 writes byte for byte what the emulator writes for the same input: the CPU-side kernel tests and the hardware
     # run the same algorithm (round trips are asserted unconditionally inside _dense_digests)

@@ -1,6 +1,7 @@
 """JNI glue (jni/tsgpu_jni.c): compiled as it stands against a test-only stand-in for <jni.h> and driven through a fake
 JNIEnv by tests/cpp/test_jni_shim.c (copy-in/copy-out array semantics, exception mapping, round trip checked by the
 oracle); plus a check that every `native` method TsGpu.java declares has its Java_* export with the right arity."""
+import json
 import os
 import re
 import subprocess
@@ -43,17 +44,14 @@ def test_java_native_declarations_match_the_exports():
 
 
 def test_java_sources_reference_only_existing_reference_members():
-    """No JDK here, so the Java cannot be compiled: at least every reference type / member the sources name must exist in
-    /root/reference when it is present (skipped on the GPU box)."""
-    ref = "/root/reference/core/src/main/java/io/aiven/kafka/tieredstorage"
-    if not os.path.isdir(ref):
-        import pytest
-        pytest.skip("reference tree not present")
-    chunk = open(os.path.join(ref, "Chunk.java")).read()
+    """The Java cannot be compiled without a JDK: at least every reference type / member the sources name must exist in
+    the reference, whose declarations tests/golden/reference_vectors.json carries (java_api, transcribed with file:line)."""
+    files = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_vectors.json")))["java_api"]["files"]
+    ref = {f: "\n".join(e["declarations"]) for f, e in files.items()}
+    chunk = ref["M/Chunk.java"]
     for field in ("transformedPosition", "transformedSize", "originalSize"):
         assert re.search(r"public final int " + field, chunk)
-    assert "SecretKey dataKey();" in open(os.path.join(ref, "manifest/SegmentEncryptionMetadata.java")).read()
-    assert "InputStream getChunk(" in open(os.path.join(ref, "fetch/ChunkManager.java")).read()
-    assert "interface DetransformChunkEnumeration extends Enumeration<byte[]>" in open(os.path.join(ref, "transform/DetransformChunkEnumeration.java")).read()
-    br = open("/root/reference/storage/core/src/main/java/io/aiven/kafka/tieredstorage/storage/BytesRange.java").read()
-    assert "public static BytesRange of(final int from, final int to)" in br
+    assert "SecretKey dataKey();" in ref["M/manifest/SegmentEncryptionMetadata.java"]
+    assert "InputStream getChunk(" in ref["M/fetch/ChunkManager.java"]
+    assert "interface DetransformChunkEnumeration extends Enumeration<byte[]>" in ref["M/transform/DetransformChunkEnumeration.java"]
+    assert "public static BytesRange of(final int from, final int to)" in ref["S/storage/BytesRange.java"]
